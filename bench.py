@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MVSNeRF render hot path (BASELINE.json metric: rays/s @ 128 samples, DTU 512x640).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--mode fp32]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--mode fp32] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic rays: one full 512x640 frame
 (327 680 rays x 128 samples) per GPU rendered against a resident encoding volume -- the
@@ -17,6 +17,10 @@ roofline   : the render kernel's algorithmic FLOPs (32 178 176 per ray, SURVEY.m
              CUDA-event duration, against the measured bf16 tensor peak (MEASURED_PEAKS.json).
 cpu_baseline / --impl reference : the CPU restatement of the reference path (oracle/, PyTorch CPU,
              all host threads) on a bounded sample of the same workload.
+
+--dump-outputs DIR : after the timed steps, the frame the last one rendered (single GPU): DIR/rgb.npy [H*W, 3] and
+             DIR/depth.npy [H*W], float32.  The scene, weights and cameras are seeded, so two builds run with the
+             same arguments can be compared output for output.
 
 Multi-GPU (torchrun, one rank per GPU): rays shard across ranks, the volume is replicated, one
 NCCL all-gather of rgb+depth per step sits inside the timed region; weak scaling (one frame per
@@ -36,6 +40,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 H, W, PAD, S = 512, 640, 24, 128
@@ -367,6 +372,8 @@ def run_ours(args):
         ms_per_step, kern_list, rest_list = timed_steps(mode, 0, args.steps)
         t_wall = time.perf_counter() - t_wall0
         n_launch = launches[0]
+        # the caller's view of the last timed step; the steps below render into the same buffers
+        last_frame = (rgb.clone(), depth.clone()) if args.dump_outputs else None
         # a timed region shorter than a few sampling periods may have caught no clock sample: keep the SAME load running
         # (untimed, same number of extra steps on every rank) until the window is at least 0.4 s long
         t_region = ms_per_step * 1e-3 * args.steps                 # max over ranks: identical on every rank
@@ -602,6 +609,10 @@ def run_ours(args):
                                     "host_cpus": os.cpu_count(), "kind": "port",
                                     "sample": f"{sample} random rays of one frame x 128 samples ({dt:.1f} s), oracle "
                                               f"port of the reference path, torch CPU, best of several pool sizes"}
+        if last_frame is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, t in zip(("rgb", "depth"), last_frame):
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
         print(json.dumps(line))
     if frame is not None:
         frame.close()
@@ -664,7 +675,13 @@ def main():
     ap.add_argument("--no-torch-gpu", action="store_true")
     ap.add_argument("--no-finetune", action="store_true")
     ap.add_argument("--no-assembly-comparison", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's rgb and depth as DIR/rgb.npy, DIR/depth.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs writes the frame of a single-GPU run of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)

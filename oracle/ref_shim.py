@@ -5,8 +5,9 @@ Loader for the *unmodified* reference (apchenstu/mvsnerf, mounted read-only at
 
   1. `tests/golden/make_golden.py` imports the reference through this shim to
      produce the committed golden vectors under tests/golden/.
-  2. `tests/test_oracle_pins.py` (CPU, only when /root/reference exists) checks
-     the restatement in `oracle/mvsnerf_oracle.py` against the live reference.
+  2. `tests/golden/make_golden_pins.py` records, the same way, what
+     `tests/test_oracle_pins.py` checks the restatement in
+     `oracle/mvsnerf_oracle.py` against.
 
 Nothing here travels to the GPU box as a dependency: /root/reference does not
 exist there and every caller must guard on `reference_available()`.

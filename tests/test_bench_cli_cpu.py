@@ -49,6 +49,16 @@ def test_product_arm_has_no_cpu_fallback():
     assert not any(l.lstrip().startswith("{") for l in r.stdout.splitlines())
 
 
+def test_steps_and_dump_outputs_arguments_are_checked():
+    for args, msg in ((["--steps", "0"], "--steps must be at least 1"),
+                      (["--gpus", "2", "--dump-outputs", "dump"], "--dump-outputs"),
+                      (["--impl", "reference", "--dump-outputs", "dump"], "--dump-outputs")):
+        r = run(args, timeout=300)
+        assert r.returncode == 2 and msg in r.stderr, (args, r.stderr[-2000:])
+        assert r.stdout.strip() == ""
+    assert not os.path.exists(os.path.join(ROOT, "dump"))
+
+
 def test_clock_sampler_uses_only_lines_that_arrived_inside_the_window(tmp_path, monkeypatch):
     """The `clocks` object of the bench line: a stand-in nvidia-smi that needs 0.2 s to come up and then streams a line
     every 25 ms; only lines stamped inside [begin(), end()] count, a window that closes before the first line reports
